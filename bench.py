@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- forward+backward rendered images/s through the drop-in SoftRenderer (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config C2|C3|C5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config C2|C3|C5] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" = one pass of the hot path over one batch of synthetic input (SURVEY.md §8d, config C2 by
@@ -264,7 +264,14 @@ class Workload:
         # lives inside the captured graph; an NCCL fallback is issued after the replay (finish()).
         if reduce or self.reduce_in_graph:
             self.reducer.reduce()
-        return loss
+        # what a caller of the step receives: the loss, the rendered images and the gradients of the trained tensors.
+        # Detached: a returned tensor that kept this step's autograd graph alive would break the next graph capture.
+        out = {"loss": loss.detach(), "images": images.detach(), "grad_mean_shape": self.mean_shape.grad}
+        if self.full:
+            out["grad_texture_flow"] = self.flow.grad
+        else:
+            out["grad_texture"] = self.texture.grad
+        return out
 
     def finish(self):
         """The part of a step that stays outside the CUDA graph: only the NCCL fallback of the all-reduce."""
@@ -284,10 +291,11 @@ class Workload:
             self._prefetch(i, cur)
         k = i % 2
         cur.wait_event(self._copied[k])
-        loss = self.step(self.stage2[k], world)
+        out = self.step(self.stage2[k], world)
         self._consumed[k].record(cur)
         self._prefetch(i + 1, cur)
-        return float(loss.item())                    # D2H read of the step's result
+        float(out["loss"].item())                    # D2H read of the step's result
+        return out
 
     def _init_e2e_pipeline(self):
         import torch
@@ -314,9 +322,9 @@ class Workload:
                        for k in (0, 1)]
 
     def gstep_resident(self, i, world):
-        loss = self.g_res[i % NUM_SETS]()
+        out = self.g_res[i % NUM_SETS]()
         self.finish()
-        return loss
+        return out
 
     def gstep_e2e(self, i, world):
         """e2e step with the H2D copy of step i+1 overlapped with the compute of step i: two static staging
@@ -329,11 +337,12 @@ class Workload:
             self._prefetch(i, cur)
         k = i % 2
         cur.wait_event(self._copied[k])                  # inputs of step i have landed in stage set k
-        loss = self.g_e2e2[k]()
+        out = self.g_e2e2[k]()
         self._consumed[k].record(cur)                    # stage set k may be overwritten after this point
         self.finish()
         self._prefetch(i + 1, cur)                       # H2D of step i+1 runs under the compute of step i
-        return float(loss.item())                        # D2H read of the step's result (syncs this stream)
+        float(out["loss"].item())                        # D2H read of the step's result (syncs this stream)
+        return out
 
     def _prefetch(self, i, cur):
         import torch
@@ -472,6 +481,26 @@ def reference_gpu_leg(cfg, ours_fwd_ms, ours_bwd_ms):
             "speedup_raster_kernels": (tf + tb) / (ours_fwd_ms + ours_bwd_ms) if ours_fwd_ms + ours_bwd_ms > 0 else None}
 
 
+DUMP_MAX_VALUES = 4 << 20  # per array: at most 4 arrays x 16 MB of float32 in one dump
+
+
+def write_outputs(path, outputs):
+    """Writes each output as <path>/<name>.npy (float32).  An array of more than DUMP_MAX_VALUES values is replaced by
+    the values at DUMP_MAX_VALUES positions of its flattened form, drawn with a fixed seed, in ascending order, so
+    two runs with the same arguments write the same positions.  Returns {name: {"shape", "stored"}}."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    info = {}
+    for name, a in outputs.items():
+        stored = a
+        if a.size > DUMP_MAX_VALUES:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_VALUES, replace=False))
+            stored = a.ravel()[idx]
+        np.save(os.path.join(path, name + ".npy"), stored.astype(np.float32))
+        info[name] = {"shape": list(a.shape), "stored": "all" if stored is a else "%d sampled values" % stored.size}
+    return info
+
+
 def run_gpu(args, cfg):
     import torch
     rank = int(os.environ.get("RANK", "0"))
@@ -512,7 +541,7 @@ def run_gpu(args, cfg):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for i in range(K):
-            fn(W + i, world)
+            out = fn(W + i, world)
         e1.record()
         barrier()
         raster.set_profile_sink(None)
@@ -523,23 +552,23 @@ def run_gpu(args, cfg):
             t = torch.tensor([ms], device=device, dtype=torch.float64)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        return ms, launches, clocks, sink
+        return ms, launches, clocks, sink, out
 
     # The captured graph holds everything of the step EXCEPT the NCCL all-reduce (capturing the collective
     # hung at N=8 in testing); the collective and the scatter back into .grad are issued after each replay.
     use_graph = not args.no_graph
     # eager pass: also records the raster kernels' own durations through the C-ABI event hooks
-    ms_eager, launches, clocks_eager, sink = timed(wl.step_resident, profile=True)
+    ms_eager, launches, clocks_eager, sink, last = timed(wl.step_resident, profile=True)
     kern = raster.collect_profile(sink)  # {"fwd": [ms...], "bwd": [ms...]}
     if use_graph:
         wl.capture(world)
-        ms_res, _, clocks, _ = timed(wl.gstep_resident)
-        wl.reset_e2e()
-        ms_e2e, _, clocks_e2e, _ = timed(wl.gstep_e2e)
+        ms_res, _, clocks, _, last = timed(wl.gstep_resident)
     else:
         ms_res, clocks = ms_eager, clocks_eager
-        wl.reset_e2e()
-        ms_e2e, _, clocks_e2e, _ = timed(wl.step_e2e)
+    # the outputs of the last step of the pass `value` is measured on, copied before the next pass overwrites them
+    outputs = {k: v.detach().float().cpu().numpy() for k, v in last.items()} if args.dump_outputs else None
+    wl.reset_e2e()
+    ms_e2e, _, clocks_e2e, _, _ = timed(wl.gstep_e2e if use_graph else wl.step_e2e)
 
     B = cfg["batch"]
     total_images = B * world * K
@@ -603,6 +632,8 @@ def run_gpu(args, cfg):
                                     "frac": (fwd_b + bwd_b) * B / (ms_res / K * 1e-3) / 1e9 / peak if peak else None},
                      "other_kernels": others},
     }
+    if rank == 0 and outputs is not None:
+        out["dump_outputs"] = write_outputs(args.dump_outputs, outputs)
     if rank == 0 and world == 1 and not args.no_reference_gpu:
         try:
             out["reference_gpu"] = reference_gpu_leg(cfg, fwd_ms, bwd_ms)
@@ -646,7 +677,7 @@ def run_reference(args, cfg):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=400)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 400; 8 with --impl reference)")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="C2", choices=sorted(CONFIGS))
@@ -654,11 +685,17 @@ def main():
     ap.add_argument("--no-other-kernels", action="store_true", help="skip the loss-kernel roofline lines")
     ap.add_argument("--no-reference-gpu", action="store_true", help="skip timing baseline/_ref (the reference's CUDA kernels)")
     ap.add_argument("--no-graph", action="store_true", help="time the eager step instead of its CUDA-graph replay")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the loss, images and gradients of the last timed step "
+                    "as DIR/<name>.npy (float32; arrays above %d values as a fixed seeded sample)" % DUMP_MAX_VALUES)
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 8 if args.impl == "reference" else 400  # each CPU step of the reference arm takes ~1 s
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path only")
     cfg = dict(CONFIGS[args.config], name=args.config)
     if args.impl == "reference":
-        if args.steps > 8:
-            args.steps = 8  # bounded: each CPU step is ~1 s
         run_reference(args, cfg)
     else:
         run_gpu(args, cfg)

@@ -1,6 +1,6 @@
 """CPU tests of the oracle (no GPU): oracle B (our restatement) is pinned
-(1) bit-exactly against oracle A = the reference's own device code compiled for the host, wherever
-    oracle/_ref is available (build container; the prebuilt .so also travels to the GPU box),
+(1) bit-exactly against oracle A = the reference's own device code compiled for the host, through its outputs
+    recorded in tests/golden/reference_host.npz (tests/golden/make_golden.py runs the same cases through oracle A),
 (2) against the committed golden vectors generated from oracle A (tests/golden/make_golden.py),
 (3) by finite differences for the one deliberate difference (texel gradient, App. B-1),
 (4) by domain invariants."""
@@ -11,11 +11,11 @@ import numpy as np
 import pytest
 
 import softras
-from util import rel_report, scene
+from util import GOLDEN as GOLDEN_DIR, assert_exact, golden_sample, rel_report, scene
 
-GOLDEN = sorted(glob.glob(os.path.join(os.path.dirname(__file__), "golden", "*.npz")))
+GOLDEN = sorted(glob.glob(os.path.join(GOLDEN_DIR, "*_t[0-9].npz")))
+REFERENCE_HOST = os.path.join(GOLDEN_DIR, "reference_host.npz")
 UMR = dict(sigma_val=1e-5, dist_eps=1e-10, gamma_val=1e-4)
-need_a = pytest.mark.skipif(not softras.have_oracle_a(), reason="oracle A (reference on host) not built")
 
 
 @pytest.mark.parametrize("path", GOLDEN, ids=[os.path.basename(p)[:-4] for p in GOLDEN])
@@ -34,40 +34,49 @@ def test_oracle_b_matches_golden_vectors(path):
         assert np.array_equal(gt, z["grad_textures"])
 
 
-@need_a
+BIT_EXACT_CASES = [(rgb, aa, isz, tr) for aa, isz, tr in [(True, 32, 2), (False, 50, 1)] for rgb in ["softmax", "hard"]]
+RANDOMISED_SEEDS = range(8)
+OTHER_MODES = [("barycentric", "sum"), ("hard", "hard"), ("euclidean", "sum")]
+
+
+def bit_exact_case(impl, rgb, aa, isz, tr):
+    """Outputs of one render + backward through oracle `impl`; make_golden.py records them for impl="A"."""
+    fv, tex = scene(2, 3, tr, seed=21)
+    img, fwd, cfg = softras.render(fv, tex, isz, anti_aliasing=aa, impl=impl, nthreads=1, aggr_func_rgb=rgb, **UMR)
+    g = np.random.default_rng(5).normal(size=img.shape).astype(np.float32)
+    gf, gt = softras.render_backward(fwd, cfg, g, anti_aliasing=aa, impl=impl, nthreads=1)
+    out = {k: fwd[k] for k in ("soft_colors", "aggrs_info", "faces_info", "p2f_info")}
+    out.update(images=img, grad_faces=gf)
+    if tr == 1:  # T2 == 1: the reference's UB cannot matter
+        out["grad_textures"] = gt
+    return out
+
+
+def other_modes_case(impl, dist, alpha):
+    fv, tex = scene(1, 2, 1, seed=22)
+    cfg = softras.RasterCfg(48, dist_func=dist, aggr_func_alpha=alpha, dist_eps=1e-4, sigma_val=1e-4)
+    fwd = softras.forward(fv, tex, cfg, impl=impl, nthreads=1)
+    g = np.random.default_rng(6).normal(size=fwd["soft_colors"].shape).astype(np.float32)
+    gf, _ = softras.backward(fwd, g, cfg, impl=impl, nthreads=1)
+    return dict(soft_colors=fwd["soft_colors"], aggrs_info=fwd["aggrs_info"], grad_faces=gf)
+
+
 @pytest.mark.parametrize("rgb", ["softmax", "hard"])
 @pytest.mark.parametrize("aa,isz,tr", [(True, 32, 2), (False, 50, 1)])
 def test_oracle_b_bit_exact_with_reference_on_host(rgb, aa, isz, tr):
-    fv, tex = scene(2, 3, tr, seed=21)
-    out = {}
-    for impl in "AB":
-        img, fwd, cfg = softras.render(fv, tex, isz, anti_aliasing=aa, impl=impl, nthreads=1, aggr_func_rgb=rgb, **UMR)
-        g = np.random.default_rng(5).normal(size=img.shape).astype(np.float32)
-        gf, gt = softras.render_backward(fwd, cfg, g, anti_aliasing=aa, impl=impl, nthreads=1)
-        out[impl] = (img, fwd, gf, gt)
-    a, b = out["A"], out["B"]
-    assert np.array_equal(a[0], b[0])
-    for k in ("soft_colors", "aggrs_info", "faces_info", "p2f_info"):
-        assert np.array_equal(a[1][k], b[1][k]), k
-    assert np.array_equal(a[2], b[2])
-    if tr == 1:  # T2 == 1: the reference's UB cannot matter
-        assert np.array_equal(a[3], b[3])
+    z = np.load(REFERENCE_HOST)
+    for k, v in bit_exact_case("B", rgb, aa, isz, tr).items():
+        assert_exact(z, "bit_exact/%s_%s_%d_%d/%s" % (rgb, aa, isz, tr, k), v)
 
 
-@need_a
 def test_other_modes_match_reference_on_host():
     """Modes UMR does not use (barycentric / hard distance, sum / hard alpha): restated too."""
-    fv, tex = scene(1, 2, 1, seed=22)
-    for dist, alpha in [("barycentric", "sum"), ("hard", "hard"), ("euclidean", "sum")]:
-        res = {}
-        for impl in "AB":
-            cfg = softras.RasterCfg(48, dist_func=dist, aggr_func_alpha=alpha, dist_eps=1e-4, sigma_val=1e-4)
-            fwd = softras.forward(fv, tex, cfg, impl=impl, nthreads=1)
-            g = np.random.default_rng(6).normal(size=fwd["soft_colors"].shape).astype(np.float32)
-            gf, _ = softras.backward(fwd, g, cfg, impl=impl, nthreads=1)
-            res[impl] = (fwd["soft_colors"], fwd["aggrs_info"], gf)
-        for x, y in zip(res["A"], res["B"]):
-            ok, msg = rel_report("%s/%s" % (dist, alpha), y, x, 1e-6, 1e-7)
+    z = np.load(REFERENCE_HOST)
+    for dist, alpha in OTHER_MODES:
+        for k, v in other_modes_case("B", dist, alpha).items():
+            key = "other_modes/%s_%s/%s" % (dist, alpha, k)
+            got, ref = golden_sample(z, key, v, 1e-6, 1e-7)
+            ok, msg = rel_report(key, got, ref, 1e-6, 1e-7)
             assert ok, msg
 
 
@@ -152,11 +161,7 @@ def test_empty_and_degenerate_inputs():
     assert np.isfinite(img).all()
 
 
-@need_a
-@pytest.mark.parametrize("seed", range(8))
-def test_randomised_configurations_match_reference_on_host(seed):
-    """Random sweep over the scalar arguments of soft_rasterize (sizes, softness, clipping planes, culling,
-    background): restatement == reference-on-host, bit for bit (single-threaded, T2 == 1 for grad_textures)."""
+def randomised_case(impl, seed):
     rng = np.random.default_rng(1000 + seed)
     B = int(rng.integers(1, 3))
     subdiv = int(rng.integers(0, 3))
@@ -168,14 +173,23 @@ def test_randomised_configurations_match_reference_on_host(seed):
               background_color=tuple(float(x) for x in rng.uniform(0, 1, 3)),
               aggr_func_rgb=str(rng.choice(["softmax", "hard"])))
     fv, tex = scene(B, subdiv, tex_res, seed=2000 + seed)
-    res = {}
-    for impl in "AB":
-        cfg = softras.RasterCfg(S, **kw)
-        fwd = softras.forward(fv, tex, cfg, impl=impl, nthreads=1)
-        g = np.random.default_rng(seed).normal(size=fwd["soft_colors"].shape).astype(np.float32)
-        gf, gt = softras.backward(fwd, g, cfg, impl=impl, nthreads=1)
-        res[impl] = (fwd["soft_colors"], fwd["aggrs_info"], fwd["p2f_info"], gf, gt)
-    for k, (x, y) in enumerate(zip(res["A"], res["B"])):
-        if k == 4 and tex_res != 1:
-            continue  # reference UB (App. B-1)
-        assert np.array_equal(x, y), "output %d differs for %r" % (k, kw)
+    cfg = softras.RasterCfg(S, **kw)
+    fwd = softras.forward(fv, tex, cfg, impl=impl, nthreads=1)
+    g = np.random.default_rng(seed).normal(size=fwd["soft_colors"].shape).astype(np.float32)
+    gf, gt = softras.backward(fwd, g, cfg, impl=impl, nthreads=1)
+    out = {k: fwd[k] for k in ("soft_colors", "aggrs_info", "p2f_info")}
+    out["grad_faces"] = gf
+    if tex_res == 1:  # reference UB (App. B-1) otherwise
+        out["grad_textures"] = gt
+    return out, kw
+
+
+@pytest.mark.parametrize("seed", RANDOMISED_SEEDS)
+def test_randomised_configurations_match_reference_on_host(seed):
+    """Random sweep over the scalar arguments of soft_rasterize (sizes, softness, clipping planes, culling,
+    background): restatement == reference-on-host, bit for bit (single-threaded, T2 == 1 for grad_textures)."""
+    z = np.load(REFERENCE_HOST)
+    out, kw = randomised_case("B", seed)
+    print("configuration:", kw)
+    for k, v in out.items():
+        assert_exact(z, "randomised/%d/%s" % (seed, k), v)

@@ -1,6 +1,6 @@
-"""Three-way gate on the B200 (SURVEY.md §8c): our kernels vs THE REFERENCE'S OWN CUDA kernels, rebuilt
-for sm_100a from /root/reference by baseline/build_ref_gpu.py (the built modules travel in
-baseline/_ref/; skipped when they are absent).
+"""Three-way gate on the B200 (SURVEY.md §8c): our kernels vs THE REFERENCE'S OWN CUDA kernels, rebuilt for sm_100a
+by baseline/build_ref_gpu.py and run on a B200 by tests/golden/make_golden.py --reference-gpu, which records their
+outputs for the cases below in tests/golden/reference_gpu.npz.
 
 * vs the -fmad=false build: the pixel planes (RGBA, softmax sum/max, hard depth/face-id) are BIT-EXACT --
   same IEEE operation sequence, same device expf; p2f / gradients differ only by float-atomics order.
@@ -13,87 +13,82 @@ import sys
 import numpy as np
 import pytest
 import torch
-import torch.nn.functional as F
 
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tools"))
 import ref_gpu_compare as rc  # noqa: E402
 from umr_b200 import raster  # noqa: E402
+from util import GOLDEN, assert_exact, golden_sample  # noqa: E402
 
 pytestmark = pytest.mark.gpu
 KW = dict(sigma_val=1e-5, dist_eps=1e-10, gamma_val=1e-4, anti_aliasing=True)
+REFERENCE_GPU = os.path.join(GOLDEN, "reference_gpu.npz")
+
+# Cases run through the reference's -fmad=false build.
+# key: (batch, tex_res, seed, icosphere subdiv, image_size, rgb_name, rgb, compare grad_textures)
+CASES = {"is128_%s_t%d" % (n, r): (2, r, 5, 3, 128, n, c, False) for n, c in (("softmax", 1), ("hard", 0)) for r in (1, 3)}
+# BASELINE config 2 per-image shape: F=1280, 256^2 (S=512), T^2=36, B=2
+CASES.update({"c2_%s" % n: (2, 6, 3, 3, 256, n, c, False) for n, c in (("softmax", 1), ("hard", 0))})
+# BASELINE config 5 per-image shape: F=5120 (icosphere subdiv 4), 1024^2 (S=2048), B=1.  T^2 == 1: the reference's
+# texel-gradient UB (App. B-1) coincides with the intended semantics, so grad_textures is compared too.
+CASES.update({"c5_softmax_t1": (1, 1, 9, 4, 1024, "softmax", 1, True), "c5_hard_t2": (1, 2, 9, 4, 1024, "hard", 0, False)})
+# Face-index plane of the reference's default (FMA-contracted) build: (batch, tex_res, seed, image_size)
+FMA_FACE_INDEX = (2, 2, 6, 128)
 
 
-def _mods():
-    return rc.load("soft_rasterize_ref"), rc.load("soft_rasterize_ref_nofma")
+def inputs(key):
+    """Seeded face vertices, textures and image gradient of a case, on the GPU."""
+    B, tex_res, seed, subdiv, IS = CASES[key][:5]
+    fv, tex = rc.scene(B, tex_res, seed=seed, subdiv=subdiv)
+    g = torch.randn(B, 4, IS, IS, device="cuda", generator=torch.Generator(device="cuda").manual_seed(2))
+    return fv, tex, g
 
 
-@pytest.mark.skipif(_mods()[1] is None, reason="baseline/_ref/soft_rasterize_ref_nofma.so not built")
+def _three_way(key, tex_requires_grad):
+    B, tex_res, seed, subdiv, IS, rgb_name, rgb, check_tex_grad = CASES[key]
+    z = np.load(REFERENCE_GPU)
+    fv, tex, g = inputs(key)
+    a = fv.clone().requires_grad_(True)
+    t = tex.clone().requires_grad_(tex_requires_grad)
+    img, p2f, aggr = raster.soft_rasterize(a, t, IS, aggr_func_rgb=rgb_name, **KW)
+    img.backward(g)
+    assert_exact(z, key + "/images", img)          # pooled RGBA
+    assert_exact(z, key + "/aggrs", aggr)          # aggregation planes
+    got, ref = golden_sample(z, key + "/p2f", p2f, 1e-4, 1e-6)
+    assert np.allclose(got, ref, rtol=1e-4, atol=1e-6)
+    grads = [("grad_faces", a.grad)] + ([("grad_textures", t.grad)] if check_tex_grad else [])
+    for name, grad in grads:
+        scale = float(z["%s/%s.absmax" % (key, name)])
+        got, ref = golden_sample(z, "%s/%s" % (key, name), grad, 1e-3, 1e-5 * scale)
+        assert np.allclose(got, ref, rtol=1e-3, atol=1e-5 * scale), name
+
+
 @pytest.mark.parametrize("rgb_name,rgb", [("softmax", 1), ("hard", 0)])
 @pytest.mark.parametrize("tex_res", [1, 3])
 def test_bit_exact_with_reference_cuda_kernels_built_without_fma(rgb_name, rgb, tex_res):
-    mod = _mods()[1]
-    IS, S = 128, 256
-    fv, tex = rc.scene(2, tex_res, seed=5)
-    a = fv.clone().requires_grad_(True)
-    img, p2f, aggr = raster.soft_rasterize(a, tex, IS, aggr_func_rgb=rgb_name, **KW)
-    g = torch.randn(img.shape, device="cuda", generator=torch.Generator(device="cuda").manual_seed(2))
-    img.backward(g)
-    colors, rp2f, raggr, finfo = rc.ref_forward(mod, fv, tex, S, rgb)
-    assert torch.equal(img.detach(), F.avg_pool2d(colors, 2, 2))
-    assert torch.equal(aggr, raggr)
-    assert torch.allclose(p2f, rp2f, rtol=1e-4, atol=1e-6)
-    ghi = (g / 4).repeat_interleave(2, dim=2).repeat_interleave(2, dim=3)
-    rgf, _ = rc.ref_backward(mod, fv, tex, colors, finfo, raggr, ghi, S, rgb)
-    scale = float(rgf.abs().max())
-    assert torch.allclose(a.grad, rgf, rtol=1e-3, atol=1e-5 * scale)
+    _three_way("is128_%s_t%d" % (rgb_name, tex_res), False)
 
 
-def _three_way(mod, fv, tex, IS, rgb_name, rgb, check_tex_grad):
-    S = 2 * IS
-    a = fv.clone().requires_grad_(True)
-    t = tex.clone().requires_grad_(True)
-    img, p2f, aggr = raster.soft_rasterize(a, t, IS, aggr_func_rgb=rgb_name, **KW)
-    g = torch.randn(img.shape, device="cuda", generator=torch.Generator(device="cuda").manual_seed(2))
-    img.backward(g)
-    colors, rp2f, raggr, finfo = rc.ref_forward(mod, fv, tex, S, rgb)
-    assert torch.equal(img.detach(), F.avg_pool2d(colors, 2, 2)), "pooled RGBA not bit-exact"
-    assert torch.equal(aggr, raggr), "aggregation planes not bit-exact"
-    assert torch.allclose(p2f, rp2f, rtol=1e-4, atol=1e-6)
-    ghi = (g / 4).repeat_interleave(2, dim=2).repeat_interleave(2, dim=3)
-    rgf, rgt = rc.ref_backward(mod, fv, tex, colors, finfo, raggr, ghi, S, rgb)
-    scale = float(rgf.abs().max())
-    assert torch.allclose(a.grad, rgf, rtol=1e-3, atol=1e-5 * scale)
-    if check_tex_grad:  # T^2 == 1: the reference's texel-gradient UB (App. B-1) coincides with the intended semantics
-        assert torch.allclose(t.grad, rgt, rtol=1e-3, atol=1e-5 * float(rgt.abs().max()))
-
-
-@pytest.mark.skipif(_mods()[1] is None, reason="baseline/_ref/soft_rasterize_ref_nofma.so not built")
 @pytest.mark.parametrize("tile", [16, 32])
 @pytest.mark.parametrize("rgb_name,rgb", [("softmax", 1), ("hard", 0)])
 def test_bit_exact_at_c2_shape(rgb_name, rgb, tile, monkeypatch):
     """BASELINE config 2 per-image shape: F=1280, 256^2 (S=512), T^2=36, B=2 -- through both forward kernels."""
     monkeypatch.setattr(raster, "FORWARD_TILE", tile)
-    fv, tex = rc.scene(2, 6, seed=3)
-    _three_way(_mods()[1], fv, tex, 256, rgb_name, rgb, False)
+    _three_way("c2_%s" % rgb_name, True)
 
 
-@pytest.mark.skipif(_mods()[1] is None, reason="baseline/_ref/soft_rasterize_ref_nofma.so not built")
 @pytest.mark.parametrize("rgb_name,rgb,tex_res", [("softmax", 1, 1), ("hard", 0, 2)])
 def test_bit_exact_at_c5_shape(rgb_name, rgb, tex_res):
     """BASELINE config 5 per-image shape: F=5120 (icosphere subdiv 4), 1024^2 (S=2048), B=1 -- the only shape
     where the cull boxes span several staging pieces and tiles carry long face lists."""
-    fv, tex = rc.scene(1, tex_res, seed=9, subdiv=4)
-    assert fv.shape[1] == 5120
-    _three_way(_mods()[1], fv, tex, 1024, rgb_name, rgb, tex_res == 1)
+    _three_way("c5_%s_t%d" % (rgb_name, tex_res), True)   # the recorded grad_faces shape pins F = 5120
 
 
-@pytest.mark.skipif(_mods()[0] is None, reason="baseline/_ref/soft_rasterize_ref.so not built")
 def test_face_index_plane_against_reference_as_normally_compiled():
-    mod = _mods()[0]
-    IS, S = 128, 256
-    fv, tex = rc.scene(2, 2, seed=6)
+    B, tex_res, seed, IS = FMA_FACE_INDEX
+    fv, tex = rc.scene(B, tex_res, seed=seed)
     _, _, aggr = raster.soft_rasterize(fv, tex, IS, aggr_func_rgb="hard", **KW)
-    _, _, raggr, _ = rc.ref_forward(mod, fv, tex, S, 0)
-    mism = int((aggr[:, 1] != raggr[:, 1]).sum())
+    ref = torch.from_numpy(np.load(REFERENCE_GPU)["fma/face_index"].astype(np.float32)).cuda()
+    assert ref.shape == aggr[:, 1].shape
+    mism = int((aggr[:, 1] != ref).sum())
     print("face-id mismatches vs FMA-compiled reference: %d / %d" % (mism, aggr[:, 1].numel()))
     assert mism <= 8  # exact ties / sliver faces only (App. B-15)
